@@ -2,6 +2,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this engine (one process per GPU; torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K ...  # the UNMODIFIED reference (oracle/_ref copy) on the host cores
+    python bench.py ... --dump-outputs DIR                   # also write what the timed path computed in its last step to DIR/*.npy
 
 A "step" = one pass of the hot path (AttModel._sample_beam: prologue + 20 timesteps + beam bookkeeping) over one batch of
 synthetic inputs (configs[1]: batch 256 per GPU).  Images are independent, so ranks shard the work with no data-path
@@ -20,6 +21,9 @@ collective ("scaling": "weak"); the only collectives are the timing barrier and 
 Other workloads (--workload): transformer_beam / aoa_beam (BASELINE configs[2] shape and AoANet decode), updown_scst / aoa_scst (SCST
 training step incl. H2D, the single NCCL gradient all-reduce and Adam; aoa_scst = BASELINE configs[3]).  The GPU arms build their
 seeded random-init model and features from imagecaptioning.pytorch_b200.synthetic; only cpu_reference_rate() / cpu_reference_scst_rate() touch oracle/.
+
+The benchmark runs the library __graft_entry__.build() made and writes nothing into the tree, which may be read-only.  With the same
+arguments every run sees the same inputs and random draws, so the arrays --dump-outputs writes can be compared between two builds.
 """
 from __future__ import annotations
 
@@ -33,6 +37,11 @@ import time
 
 REPO = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, REPO)
+sys.dont_write_bytecode = True          # no __pycache__ in the tree
+
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_LOGPROB_ROWS = 32                  # seeded sample of the [rows, T, V+1] log-prob rows written by --dump-outputs
+DUMP_GRAD_ENTRIES = 1 << 20             # seeded sample of the SCST step's gradient entries
 
 CFG = dict(V=9487, E=1000, H=1000, A=512, F_fc=2048, F_att=2048, T=20)     # configs/updown/updown.yml + opts.py defaults
 R = 36
@@ -51,7 +60,14 @@ def parse():
     p.add_argument('--no-cpu-baseline', action='store_true')
     p.add_argument('--workload', default='updown_beam', choices=['updown_beam', 'transformer_beam', 'aoa_beam', 'updown_scst', 'aoa_scst', 'transformer_scst'],
                    help='updown_beam = BASELINE.json configs[1] (the headline); transformer_beam = configs[2] (use --batch 64); aoa_beam = AoANet decode')
+    p.add_argument('--dump-outputs', metavar='DIR', default=None,
+                   help='after the timed steps, write what each timed path computed in its last step to DIR/<name>.npy (float32 / float64, '
+                        'seeded samples of the large arrays, at most 64 MB in all)')
     args = p.parse_args()
+    if args.steps < 1:
+        p.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        p.error('--dump-outputs writes the outputs of the GPU arm (--impl b200)')
     if args.batch is None:
         args.batch = 10 if args.workload in ('updown_scst', 'aoa_scst', 'transformer_scst') else 256
     return args
@@ -204,11 +220,43 @@ def _per_rank(ms, dev, world):
     return vals, max(vals)
 
 
+def _seeded_subset(n, k, seed=0):
+    """Sorted indices of a fixed, seeded choice of min(n, k) of range(n)."""
+    import numpy as np
+    import torch
+    return torch.from_numpy(np.sort(np.random.default_rng(seed).choice(n, size=min(n, k), replace=False)))
+
+
+def decode_outputs(prefix, seq, logprobs):
+    """What a caller of the decode receives: the caption ids [B, T] and a seeded sample of the log-prob rows [B, T, V+1]."""
+    out = {prefix + '_seq': seq.cpu()}
+    if logprobs is not None:
+        rows = _seeded_subset(logprobs.shape[0], DUMP_LOGPROB_ROWS)
+        out[prefix + '_logprobs_sample'] = logprobs[rows.to(logprobs.device)].cpu()
+        out[prefix + '_logprobs_sample_rows'] = rows
+    return out
+
+
+def write_outputs(out_dir, arrays):
+    """DIR/<name>.npy per array: integer and float64 arrays as float64, the rest as float32."""
+    import numpy as np
+    host = {}
+    for name, a in arrays.items():
+        a = np.asarray(a.detach().cpu().numpy() if hasattr(a, 'detach') else a)
+        host[name] = a.astype(np.float64 if a.dtype == np.float64 or np.issubdtype(a.dtype, np.integer) else np.float32)
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError('--dump-outputs: %d bytes exceed the %d byte limit' % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 def bench_scst(args, rank, world, local_rank, dev, workload, batch):
     """SCST samples/sec (the second half of BASELINE.json's metric): AoANet (configs[3]) or UpDown, per-GPU batch `batch` images,
     train_sample_n = 5, CIDEr-D reward, greedy baseline, BPTT, gradient all-reduce over NCCL (overlapped with the backward pass when the loss
     wrapper supports it), value clipping and Adam.  Every step starts from pinned HOST features (H2D inside the timed region) and ends with
-    the D2H read of the loss.  Returns the result dict on every rank (rank 0 prints)."""
+    the D2H read of the loss.  Returns the result dict on every rank (rank 0 prints) and, with --dump-outputs, the last step's outputs."""
     import argparse as ap
     import torch
     import torch.distributed as dist
@@ -241,11 +289,14 @@ def bench_scst(args, rank, world, local_rank, dev, workload, batch):
     idx = torch.arange(B)
     grad_bytes = [0]
     ar_events = []
+    last = {}
 
     def step(i, timed=False):
         fc_h, att_h = host[i % 3]
         fc, att = fc_h.to(dev, non_blocking=True), att_h.to(dev, non_blocking=True)      # H2D every step (inputs start on the host)
         out = lw(fc, att, None, None, None, gts, idx, True, False, False)
+        if args.dump_outputs:
+            last.update(loss=out['loss'].detach(), reward=out['reward'].detach())
         optim.zero_grad(set_to_none=True)
         out['loss'].backward()
         if fused_sync:
@@ -286,6 +337,15 @@ def bench_scst(args, rank, world, local_rank, dev, workload, batch):
     sampler.stop_flag = True
     sampler.join()
     per_rank, ms = _per_rank(e0.elapsed_time(e1), dev, world)
+    dump = None
+    if args.dump_outputs:
+        # the loss and mean reward the step returns, the captions it sampled, and a seeded sample of the gradients it left (clipped by the step)
+        grads = torch.cat([p.grad.reshape(-1) for p in model.parameters() if p.grad is not None])
+        pick = _seeded_subset(grads.numel(), DUMP_GRAD_ENTRIES)
+        dump = {'scst_loss': last['loss'].reshape(1), 'scst_reward': last['reward'].reshape(1),
+                'scst_sample_seq': lw.last_step['sample_seq'], 'scst_grad_sample': grads[pick.to(dev)], 'scst_grad_sample_index': pick}
+        dump = {k: v.cpu() for k, v in dump.items()}
+        del grads
     if fused_sync:
         allreduce_ms = getattr(lw, 'last_sync_exposed_ms', None)
     else:
@@ -312,7 +372,7 @@ def bench_scst(args, rank, world, local_rank, dev, workload, batch):
                    'note': 'the timed region IS end to end: pinned host features copied H2D every step, loss read back D2H every step'}}
     del optim, lw, model
     torch.cuda.empty_cache()
-    return res
+    return res, dump
 
 
 def main():
@@ -329,7 +389,7 @@ def main():
         # configured batch; rank 0 alone runs it.
         if rank != 0:
             return
-        steps = max(1, min(args.steps, 3))
+        steps = args.steps
         batch = args.batch if args.workload == 'updown_beam' else args.cpu_batch
         rate, dt, cores, kind = cpu_reference_rate(batch, args.beam, steps, 1)
         line = {'impl': 'reference', 'metric': 'captions/sec at beam=5 seq_len=20', 'value': rate, 'unit': 'captions/s', 'n_gpus': args.gpus,
@@ -348,9 +408,9 @@ def main():
 
     import torch
     import torch.distributed as dist
-    import __graft_entry__ as ge
-    if local_rank == 0:
-        ge.build()
+    import imagecaptioning.pytorch_b200 as b200
+    b200._lib.load()                        # made by __graft_entry__.build(); a missing library is an error, not a rebuild
+    torch.manual_seed(1234 + rank)          # the SCST steps draw their sampling / dropout seeds from torch's generator
     torch.cuda.set_device(local_rank)
     try:        # bind this rank to the CPU cores next to its GPU (NUMA): the SCST step is ~1300 launches of host-side work per step
         if os.environ.get('CAPB200_BENCH_NO_AFFINITY'):
@@ -366,8 +426,10 @@ def main():
     from imagecaptioning.pytorch_b200 import synthetic as syn      # seeded random-init weights / features: the GPU arm never touches oracle/
     dev = torch.device('cuda', local_rank)
     if args.workload in ('updown_scst', 'aoa_scst', 'transformer_scst'):
-        res = bench_scst(args, rank, world, local_rank, dev, args.workload, args.batch)
+        res, dump = bench_scst(args, rank, world, local_rank, dev, args.workload, args.batch)
         if rank == 0:
+            if dump is not None:
+                write_outputs(args.dump_outputs, dump)
             line = dict(res, warmup=args.warmup, higher_is_better=True, vs_baseline=None, dtype='f32', data='synthetic', gpu_launches=res['launches'] * args.steps)
             print(json.dumps(line))
         if world > 1:
@@ -442,18 +504,25 @@ def main():
         l0 = model.launch_count
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for i in range(steps):
+        for i in range(steps - 1):
             fn(warmup + i)
+        out = fn(warmup + steps - 1)         # kept for --dump-outputs; earlier outputs are freed as before
         e1.record()
         barrier()
         sampler.stop_flag = True
         sampler.join()
         per_rank, mx = _per_rank(e0.elapsed_time(e1), dev, world)
-        return mx, sampler.summary(), model.launch_count - l0, per_rank
+        return mx, sampler.summary(), model.launch_count - l0, per_rank, out
 
-    ms, clocks, launches, per_rank = timed(step_resident, args.steps, max(3, args.warmup))
+    dump = {}
+    ms, clocks, launches, per_rank, out = timed(step_resident, args.steps, max(3, args.warmup))
+    if args.dump_outputs:                   # copied before the next call of the model
+        dump.update(decode_outputs('decode', *out))
     value = world * B * args.steps / (ms / 1e3)
-    ms_e2e, _, _, per_rank_e2e = timed(step_e2e, args.steps, max(3, args.warmup))
+    ms_e2e, _, _, per_rank_e2e, out = timed(step_e2e, args.steps, max(3, args.warmup))
+    if args.dump_outputs:
+        dump.update(decode_outputs('e2e', out, None))
+    del out
     pending.clear()
     e2e = world * B * args.steps / (ms_e2e / 1e3)
 
@@ -465,6 +534,8 @@ def main():
                     'per_rank_ms_per_step': [v / args.steps for v in per_rank],
                     'e2e': {'value': e2e, 'unit': 'captions/s', 'h2d_bytes_per_step': B * (CFG['F_fc'] + R * CFG['F_att']) * 4, 'd2h_bytes_per_step': B * T * 8},
                     'gpu_launches': launches, 'roofline': None}
+            if args.dump_outputs:
+                write_outputs(args.dump_outputs, dump)
             print(json.dumps(line))
         if world > 1:
             dist.destroy_process_group()
@@ -517,7 +588,9 @@ def main():
     # the second half of BASELINE.json's metric, in the same line: SCST samples/sec on configs[3] (AoANet, per-GPU batch 10 x 5 samples)
     scst = None
     if not os.environ.get('CAPB200_BENCH_NO_SCST'):
-        scst = bench_scst(args, rank, world, local_rank, dev, 'aoa_scst', 10)
+        scst, scst_dump = bench_scst(args, rank, world, local_rank, dev, 'aoa_scst', 10)
+        if scst_dump is not None:
+            dump.update(scst_dump)
 
     if rank != 0:
         if world > 1:
@@ -539,6 +612,8 @@ def main():
         line['cpu_baseline'] = {'value': rate, 'unit': 'captions/s', 'cores': cores, 'kind': kind, 'host_cpus': os.cpu_count(),
                                 'sample': '2 steps of batch %d through %s (torch fp32 CPU, best thread count of a calibration sweep)' %
                                           (args.cpu_batch, 'the unmodified reference modules copied to oracle/_ref' if kind == 'reference' else 'the oracle port')}
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, dump)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -758,12 +758,34 @@ def gen_state_dict_keys(out_dir):
     print('state_dict_keys', {k: len(v) for k, v in res.items()})
 
 
+def gen_eval_split(out_dir):
+    """The reference's eval_split on the stub model / loader of tests/test_eval_cpu.py: loss, predictions and, for sample_n > 1, the
+    n_predictions it saves under eval_results/ (one run per sample_n_method)."""
+    import json
+    sys.path.insert(0, os.path.join(REPO, 'tests'))
+    import test_eval_cpu as te
+    import captioning.utils.eval_utils as E
+    cwd = os.getcwd()
+    res = {}
+    for name, kwargs in [('n1', te.EVAL_KWARGS)] + [(m, te.eval_n_kwargs(m)) for m in te.N_METHODS]:
+        os.chdir(tempfile.mkdtemp(prefix='eval_'))
+        loss, preds, _ = E.eval_split(te._StubModel(te.T, te.V1), te._crit, te._StubLoader(10, 4, te.T, te.V1), dict(kwargs))
+        res[name] = {'loss': float(loss), 'predictions': [{k: p[k] for k in ('image_id', 'caption', 'perplexity', 'entropy')} for p in preds]}
+        if kwargs['sample_n'] > 1:
+            _, n_preds = torch.load(os.path.join('eval_results', '.saved_pred_%s_val.pth' % kwargs['id']), weights_only=False)
+            res[name]['n_predictions'] = [{k: e[k] for k in ('image_id', 'caption', 'perplexity') if k in e} for e in n_preds]
+    os.chdir(cwd)
+    with open(os.path.join(out_dir, 'eval_split.json'), 'w') as f:
+        json.dump(res, f, indent=1, sort_keys=True)
+    print('eval_split', {k: len(v['predictions']) for k, v in res.items()})
+
+
 def main():
     out_dir = os.path.join(REPO, 'tests', 'golden')
     os.makedirs(out_dir, exist_ok=True)
     scratch = _enter_scratch()
     torch.set_num_threads(os.cpu_count())
-    which = sys.argv[1:] or ['small', 'newfc', 'full', 'ciderd', 'rc', 'keys', 'tfm', 'aoa', 'xe', 'dseq', 'pascal', 'penalty', 'b256', 'tfm64', 'aoafull', 'options', 'tfmtrain', 'tfmtrainfull']
+    which = sys.argv[1:] or ['small', 'newfc', 'full', 'ciderd', 'rc', 'keys', 'tfm', 'aoa', 'xe', 'dseq', 'pascal', 'penalty', 'b256', 'tfm64', 'aoafull', 'options', 'tfmtrain', 'tfmtrainfull', 'eval']
     if 'small' in which:
         gen_updown_small(out_dir)
     if 'newfc' in which:
@@ -800,6 +822,8 @@ def main():
         gen_transformer_train(out_dir, scratch)
     if 'tfmtrainfull' in which:
         gen_transformer_train_full(out_dir, scratch)
+    if 'eval' in which:
+        gen_eval_split(out_dir)
 
 
 if __name__ == '__main__':

@@ -1,5 +1,7 @@
 """CPU test of the evaluation-loop mirror (imagecaptioning.pytorch_b200/eval_utils.py): the same stub model / loader driven through the
-UNMODIFIED reference eval_split (oracle/_ref, when present) and through the mirror must give the same predictions and loss."""
+mirror must give the predictions and loss the UNMODIFIED reference eval_split gave (tests/golden/eval_split.json, made by
+oracle/make_golden.py: gen_eval_split)."""
+import json
 import os
 
 import numpy as np
@@ -67,33 +69,34 @@ def _crit(lp, target, mask):
     return -(lp.gather(2, target.unsqueeze(2)).squeeze(2) * mask).sum() / mask.sum()
 
 
-def test_eval_split_matches_the_reference_loop(tmp_path, monkeypatch):
+T, V1 = 6, 12
+EVAL_KWARGS = {'verbose': False, 'verbose_loss': 1, 'split': 'val', 'language_eval': 0, 'dataset': 'coco', 'beam_size': 1, 'sample_n': 1,
+               'device': 'cpu', 'id': 'stub', 'num_images': -1}
+N_METHODS = ['sample', 'bs', 'top3']
+
+
+def eval_n_kwargs(method):
+    return dict(EVAL_KWARGS, sample_n=3, sample_n_method=method, id='stubn')
+
+
+def _golden(golden_dir, name):
+    with open(os.path.join(golden_dir, 'eval_split.json')) as f:
+        return json.load(f)[name]
+
+
+def test_eval_split_matches_the_reference_loop(tmp_path, monkeypatch, golden_dir):
     from imagecaptioning.pytorch_b200 import eval_utils as EU
-    T, V1 = 6, 12
-    kwargs = {'verbose': False, 'verbose_loss': 1, 'split': 'val', 'language_eval': 0, 'dataset': 'coco', 'beam_size': 1, 'sample_n': 1,
-              'device': 'cpu', 'id': 'stub', 'num_images': -1}
     model = _StubModel(T, V1)
     monkeypatch.chdir(tmp_path)
-    loss, preds, stats = EU.eval_split(model, _crit, _StubLoader(10, 4, T, V1), dict(kwargs))
+    loss, preds, stats = EU.eval_split(model, _crit, _StubLoader(10, 4, T, V1), dict(EVAL_KWARGS))
     assert stats is None and len(preds) == 10 and [p['image_id'] for p in preds] == list(range(10))
     assert model.training                                     # switched back (eval_utils.py:212)
-    # against the unmodified reference loop, when its copy is present (build container and GPU box)
-    from oracle import ref_runtime as rr
-    if rr.available():
-        cwd = os.getcwd()
-        rr.enter()
-        try:
-            import captioning.utils.eval_utils as REF
-        except Exception as exc:                               # the reference loop imports optional packages (pycocoevalcap, ...)
-            os.chdir(cwd)
-            pytest.skip('reference eval_utils not importable here: %r' % (exc,))
-        os.chdir(str(tmp_path))
-        rloss, rpreds, _ = REF.eval_split(_StubModel(T, V1), _crit, _StubLoader(10, 4, T, V1), dict(kwargs))
-        os.chdir(cwd)
-        assert abs(loss - rloss) < 1e-6
-        assert [p['caption'] for p in preds] == [p['caption'] for p in rpreds]
-        assert np.allclose([p['perplexity'] for p in preds], [p['perplexity'] for p in rpreds], atol=1e-5)
-        assert np.allclose([p['entropy'] for p in preds], [p['entropy'] for p in rpreds], atol=1e-5)
+    ref = _golden(golden_dir, 'n1')
+    rpreds = ref['predictions']
+    assert abs(loss - ref['loss']) < 1e-6
+    assert [p['caption'] for p in preds] == [p['caption'] for p in rpreds]
+    assert np.allclose([p['perplexity'] for p in preds], [p['perplexity'] for p in rpreds], atol=1e-5)
+    assert np.allclose([p['entropy'] for p in preds], [p['entropy'] for p in rpreds], atol=1e-5)
 
 
 def test_prefetch_loader_is_one_batch_ahead_and_stops_at_wrap():
@@ -103,37 +106,21 @@ def test_prefetch_loader_is_one_batch_ahead_and_stops_at_wrap():
     assert seen == [0, 4, 8] and loader.calls == 3             # the wrapped batch is the last one fetched
 
 
-@pytest.mark.parametrize('method', ['sample', 'bs', 'top3'])
-def test_eval_split_n_matches_the_reference_loop(tmp_path, monkeypatch, method):
+@pytest.mark.parametrize('method', N_METHODS)
+def test_eval_split_n_matches_the_reference_loop(tmp_path, monkeypatch, golden_dir, method):
     """sample_n > 1 (eval_utils.py:196-197 -> eval_split_n): sample_n captions per image through 'bs' (the best beams) and the sampling
     methods, n_predictions sorted by perplexity and saved beside the predictions like the reference does."""
     from imagecaptioning.pytorch_b200 import eval_utils as EU
-    T, V1 = 6, 12
-    kwargs = {'verbose': False, 'verbose_loss': 1, 'split': 'val', 'language_eval': 0, 'dataset': 'coco', 'beam_size': 1, 'sample_n': 3,
-              'sample_n_method': method, 'device': 'cpu', 'id': 'stubn', 'num_images': -1}
     monkeypatch.chdir(tmp_path)
-    loss, preds, _ = EU.eval_split(_StubModel(T, V1), _crit, _StubLoader(10, 4, T, V1), dict(kwargs))
+    loss, preds, _ = EU.eval_split(_StubModel(T, V1), _crit, _StubLoader(10, 4, T, V1), eval_n_kwargs(method))
     saved_preds, saved_n = torch.load(os.path.join('eval_results', '.saved_pred_stubn_val.pth'), weights_only=False)
     assert len(saved_preds) == 10 and len(saved_n) == 3 * 12          # three batches of four images reach eval_split_n (the loop's own bookkeeping)
     if method != 'bs':
         ps = [e['perplexity'] for e in saved_n]
         assert ps == sorted(ps)
-    from oracle import ref_runtime as rr
-    if rr.available():
-        cwd = os.getcwd()
-        rr.enter()
-        try:
-            import captioning.utils.eval_utils as REF
-        except Exception as exc:
-            os.chdir(cwd)
-            pytest.skip('reference eval_utils not importable here: %r' % (exc,))
-        ref_dir = tmp_path / 'ref'
-        ref_dir.mkdir()
-        os.chdir(str(ref_dir))
-        rloss, rpreds, _ = REF.eval_split(_StubModel(T, V1), _crit, _StubLoader(10, 4, T, V1), dict(kwargs))
-        _, rn = torch.load(os.path.join('eval_results', '.saved_pred_stubn_val.pth'), weights_only=False)
-        os.chdir(cwd)
-        assert abs(loss - rloss) < 1e-6 and [p['caption'] for p in preds] == [p['caption'] for p in rpreds]
-        assert [(e['image_id'], e['caption']) for e in saved_n] == [(e['image_id'], e['caption']) for e in rn]
-        if method != 'bs':
-            assert np.allclose([e['perplexity'] for e in saved_n], [e['perplexity'] for e in rn], atol=1e-5)
+    ref = _golden(golden_dir, method)
+    rpreds, rn = ref['predictions'], ref['n_predictions']
+    assert abs(loss - ref['loss']) < 1e-6 and [p['caption'] for p in preds] == [p['caption'] for p in rpreds]
+    assert [(e['image_id'], e['caption']) for e in saved_n] == [(e['image_id'], e['caption']) for e in rn]
+    if method != 'bs':
+        assert np.allclose([e['perplexity'] for e in saved_n], [e['perplexity'] for e in rn], atol=1e-5)
